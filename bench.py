@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- DISGAT fwd+bwd edges/s on B200 (the BASELINE.json metric).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl edis|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl edis|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = DISGAT.get_em forward + backward of a scalar loss, 2 layers x C channels, train
@@ -33,6 +33,8 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+DUMP_BYTES = 64_000_000
+NPY_HEADER = 4096                                  # allowance per .npy file for its header
 
 
 def parse():
@@ -59,9 +61,19 @@ def parse():
     ap.add_argument("--max-chunk", type=int, default=0)
     ap.add_argument("--no-epoch-metric", action="store_true", help="skip the cora_full epoch-ms secondary metric")
     ap.add_argument("--no-ssl-metric", action="store_true", help="skip the SupEdge step secondary metric")
-    ap.add_argument("--cache-dir", default=os.environ.get("EDIS_CACHE_DIR", os.path.join(ROOT, ".cache")),
-                    help="graph cache directory ('' = no cache)")
+    # no cache unless asked for: a run writes nothing into the (possibly read-only) source tree and leaves no
+    # GB-sized graph files behind, and every run builds its graph with the code under test
+    ap.add_argument("--cache-dir", default=os.environ.get("EDIS_CACHE_DIR", ""),
+                    help="graph cache directory kept between runs (default: none; the graph is generated in every "
+                         "run, by every rank at N > 1)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write what the last of the --steps timed steps behind `value` computed to DIR/<name>.npy "
+                         "(float32): "
+                         "get_em's two embeddings at a fixed seeded sample of rows, the loss and every parameter "
+                         "gradient, at most %d bytes in all" % DUMP_BYTES)
     a = ap.parse_args()
+    if a.steps < 1:
+        ap.error("--steps must be at least 1")
     base = {"A": (2_400_000, 30_600_000, 100), "B": (10_000_000, 246_000_000, 64)}[a.config]
     a.nodes = a.nodes or base[0]
     a.raw_edges = a.raw_edges or base[1]
@@ -318,8 +330,9 @@ def _gen_key(a):
 
 
 def global_graph_indices(a, rank, world, dev="cuda"):
-    """[2, E] processed adjacency of the ONE bench graph, generated once per box (rank 0) and shared
-    with the other ranks / later runs through the cache directory as a memory-mapped .npy.
+    """[2, E] processed adjacency of the ONE bench graph.  With a cache directory it is generated once per box
+    (rank 0) and shared with the other ranks / later runs as a memory-mapped .npy; without one (or when it cannot
+    be written) every rank generates it from the same seed.
     Every decision that changes which collectives run is taken by rank 0 and broadcast, so ranks that
     arrive at different times cannot take different branches."""
     from edgedisentangle_ssl_b200.synthetic import power_law_graph
@@ -352,6 +365,31 @@ def global_graph_indices(a, rank, world, dev="cuda"):
     if idx is None:
         idx = np.load(path, mmap_mode="r") if saved else power_law_graph(a.nodes, a.raw_edges, seed=0)
     return idx, False
+
+
+def dump_row_bytes(grad_numels, n_feats):
+    """Bytes --dump-outputs has left for embedding rows next to the loss, the gradients and every file's header."""
+    return DUMP_BYTES - 4 - 4 * sum(grad_numels) - (1 + len(grad_numels) + n_feats) * NPY_HEADER
+
+
+def dump_outputs(out_dir, last, n_total, lo):
+    """--dump-outputs: what the last timed step returned to its caller, as float32 .npy files.  The rows of
+    get_em's two [N, D] embeddings are a sample drawn with a fixed seed over the global row ids, as many as fit
+    DUMP_BYTES next to the loss and the gradients, so runs with the same arguments write the same rows; with
+    several ranks, rank 0 writes the sampled rows of its own range."""
+    arrays = {"loss": last["loss"].reshape(1)}
+    arrays.update(("grad." + name, g) for name, g in last["grads"])
+    feats = last["feats"]
+    room = dump_row_bytes([g.numel() for _, g in last["grads"]], len(feats))
+    k = min(n_total, room // (4 * sum(f.shape[1] for f in feats)))      # >= 1: checked in main() before timing
+    rows =np.sort(np.random.RandomState(0).choice(n_total, k, replace=False))
+    rows = rows[(rows >= lo) & (rows < lo + feats[0].shape[0])] - lo
+    idx = torch.from_numpy(rows).to(feats[0].device)
+    for i, f in enumerate(feats):
+        arrays["get_em_%d" % i] = f[idx]
+    os.makedirs(out_dir, exist_ok=True)
+    for name, v in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), v.detach().float().cpu().numpy())
 
 
 def main():
@@ -434,7 +472,12 @@ def main():
     enc = edis.DISGAT(margs, nfeat=a.feat, nhid=a.nhid, nclass=a.nhid, nheads=a.nhead, dropout=a.dropout).to(dev)
     fus = [edis.FuseLayer(margs, a.nhead, nfeat=a.nhid).to(dev), edis.FuseLayer(margs, a.nhead, nfeat=a.nhid).to(dev)]
     enc.train()
-    params = [p for m in [enc] + fus for p in m.parameters()]
+    named = [("encoder." + n, p) for n, p in enc.named_parameters()] + \
+        [("fuser%d.%s" % (i, n), p) for i, f in enumerate(fus) for n, p in f.named_parameters()]
+    params = [p for _, p in named]
+    # every rank decides this the same way before any timing, so no rank is left waiting at a collective
+    if a.dump_outputs and dump_row_bytes([p.numel() for p in params], 2) < 4 * 2 * a.nhid:
+        raise SystemExit("--dump-outputs: the gradients alone exceed %d bytes" % DUMP_BYTES)
     # features / loss weights: rows [lo, lo + n_local) of one global seeded stream per 64K-row block, so the
     # strong-scaling runs at every N work on the SAME node features
     def rows_of(width, seed):
@@ -468,7 +511,7 @@ def main():
             copied[b].record(copy_stream)
     loss_host = torch.zeros(1).pin_memory()
 
-    def step(from_host):
+    def step(from_host, keep=None):
         xin = x_dev
         if from_host:
             b = state["k"] % 2
@@ -484,6 +527,9 @@ def main():
         if world > 1:
             with Fn.phase("grad_allreduce"):
                 par.allreduce_grads(params)
+        if keep is not None:                       # references only: no copy, no sync inside the timed window
+            keep.update(feats=[f.detach() for f in feats], loss=loss.detach(),
+                        grads=[(n, p.grad) for n, p in named if p.grad is not None])
         if from_host:
             loss_host.copy_(loss.detach().reshape(1), non_blocking=True)
             consumed[state["k"] % 2].record(torch.cuda.current_stream())
@@ -492,12 +538,12 @@ def main():
             p.grad = None
         return loss
 
-    def timed(from_host, k):
+    def timed(from_host, k, keep=None):
         ev0, ev1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
         ev0.record()
-        for _ in range(k):
-            step(from_host)
+        for i in range(k):
+            step(from_host, keep if i == k - 1 else None)
         ev1.record()
         barrier()
         ms = ev0.elapsed_time(ev1)
@@ -513,7 +559,8 @@ def main():
     clocks.start()
     Fn.TIMER.reset()
     Fn.TIMER.enabled = True
-    ms_res = timed(False, a.steps)
+    last = {} if (a.dump_outputs and rank == 0) else None
+    ms_res = timed(False, a.steps, last)
     Fn.TIMER.enabled = False
     kernel_list = Fn.TIMER.durations_ms()
     kernel_bytes = Fn.TIMER.bytes()
@@ -525,6 +572,9 @@ def main():
     step(True)
     ms_e2e = timed(True, a.steps)
     clk = clocks.stop()
+    if last:                                       # after the clock samples: they cover GPU work only
+        dump_outputs(a.dump_outputs, last, n_total, lo)
+        del last
 
     e_total = e_local
     if world > 1:

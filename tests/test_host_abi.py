@@ -220,14 +220,15 @@ int main(void) { return table[0] == 0; }
 
 
 def test_reference_arm_runs_without_the_package():
-    """`bench.py --impl reference` (the driver's reference arm): times the UNMODIFIED reference from oracle/_ref on
-    the host cores, prints one JSON line with impl / cpu_baseline / e2e, and never maps libedis.so (it must not import
-    edgedisentangle_ssl_b200).  Tiny sample here; skipped where oracle/_ref has not been built."""
+    """`bench.py --impl reference` (the reference arm): times the UNMODIFIED reference from oracle/_ref on the host
+    cores, prints one JSON line with impl / cpu_baseline / e2e, and never maps libedis.so (it must not import
+    edgedisentangle_ssl_b200).  Tiny sample here.  The reference sources are not part of this repository: only
+    where build() found them and made oracle/_ref does this cover the unmodified reference.  Everywhere else it
+    covers the oracle-port arm (the line must say kind "port"), which shares the no-package, no-libedis property."""
     import json
     import subprocess
     import sys
-    if not os.path.exists(os.path.join(ROOT, "oracle", "_ref", "MANIFEST.json")):
-        pytest.skip("oracle/_ref not built (python oracle/make_ref.py needs /root/reference)")
+    kind = "reference" if os.path.exists(os.path.join(ROOT, "oracle", "_ref", "MANIFEST.json")) else "port"
     code = ("import sys, runpy; sys.argv = ['bench.py', '--impl', 'reference', '--steps', '1', '--warmup', '1', "
             "'--ref-total-s', '1', '--cpu-probe-edges', '20000']; runpy.run_path(%r, run_name='__main__'); "
             "mods = [m for m in sys.modules if m.startswith('edgedisentangle_ssl_b200')]; "
@@ -236,6 +237,6 @@ def test_reference_arm_runs_without_the_package():
     assert p.returncode == 0, p.stderr[-2000:]
     line = json.loads([l for l in p.stdout.splitlines() if l.startswith("{")][-1])
     assert line["impl"] == "reference" and line["unit"] == "edges/s" and line["value"] > 0
-    assert line["cpu_baseline"]["kind"] == "reference" and line["cpu_baseline"]["cores"] >= 1
+    assert line["cpu_baseline"]["kind"] == kind and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"]["h2d_bytes_per_step"] == 0 and line["gpu_launches"] == 0
     assert "LOADED [] False" in p.stdout, p.stdout[-400:]
