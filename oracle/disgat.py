@@ -53,10 +53,12 @@ def pair_logits(x, W, a, pairs, att):
     raise ValueError(att)
 
 
-def disga_layer(p, prefix, x, indices, att, gnn, dropout=0.0, training=False, aux=None):
+def disga_layer(p, prefix, x, indices, att, gnn, dropout=0.0, training=False, aux=None, keep=None):
     """One DisGALayer channel, sparse branch, incl. the ELU of `forward`.
 
     Follows layers.py:340-416 and 493-511.  `p[prefix + 'W']` etc. are the parameters.
+    `keep` ([E,1] multipliers: 0 or 1/(1-p)) replaces the dropout of alpha by a given mask, e.g. the
+    one a kernel drew, so that a train-mode result can be compared element for element.
     Returns (elu(h'), edge_e[E,1] raw logits, [aux logits]) -- aux list only if given.
     """
     n = x.size(0)
@@ -68,7 +70,10 @@ def disga_layer(p, prefix, x, indices, att, gnn, dropout=0.0, training=False, au
             aux = [aux]
         aux_out = [pair_logits(x, W, a, q, att) for q in aux]
     alpha = sp_softmax(indices, torch.sigmoid(edge_e), n)
-    alpha = F.dropout(alpha, dropout, training=training)
+    if keep is None:
+        alpha = F.dropout(alpha, dropout, training=training)
+    else:
+        alpha = alpha * keep.to(alpha.dtype)
     if gnn == "AT":
         h = sp_matmul(indices, alpha, x @ p[prefix + "W_em"])
     elif gnn == "GCN":

@@ -45,6 +45,33 @@ def assert_close(got, ref, rtol=RTOL, what="", floor=0.0):
     assert err <= rtol, "%s: rel err %.3e > %.1e" % (what, err, rtol)
 
 
+def keep_scale(seed, idx, p):
+    """Bit-exact numpy restatement of the kernels' dropout multiplier (csrc/edis_common.cuh keep_scale):
+    float32 inv_keep = 1 / (1 - p) where element `idx` is kept, 0 where it is dropped.  The layer kernels
+    draw element csr_slot * C + channel of the attention weights with the layer's 64-bit seed."""
+    idx = np.asarray(idx, dtype=np.uint64)
+    seed = np.uint64(int(seed) & (2 ** 64 - 1))
+    lo32 = np.uint64(0xFFFFFFFF)
+    u32 = lambda v: (v & lo32).astype(np.uint32)   # noqa: E731
+    with np.errstate(over="ignore"):
+        x = u32(idx) ^ u32(seed)
+        x = x * np.uint32(0x9E3779B1)
+        x ^= u32(idx >> np.uint64(32)) * np.uint32(0x85EBCA77) + u32(seed >> np.uint64(32))
+        x ^= x >> np.uint32(16)
+        x = x * np.uint32(0x85EBCA6B)
+        x ^= x >> np.uint32(13)
+        x = x * np.uint32(0xC2B2AE35)
+        x ^= x >> np.uint32(16)
+    u = (x >> np.uint32(8)).astype(np.float32) * np.float32(1.0 / 16777216.0)
+    inv_keep = np.float32(1) / (np.float32(1) - np.float32(p))
+    return np.where(u >= np.float32(p), inv_keep, np.float32(0)).astype(np.float32)
+
+
+def edge_keep(seed, e, C, p):
+    """[e, C] dropout multipliers of a layer's attention weights (CSR slot x channel)."""
+    return keep_scale(seed, np.arange(e * C, dtype=np.uint64), p).reshape(e, C)
+
+
 GRAD_FLOOR = 1e-3
 
 

@@ -210,30 +210,36 @@ def grad_tol(ref32, ref64):
     return max(RT_GRAD, 16.0 * rel_err(ref32, ref64))
 
 
-def oracle_layer_all(chs, x_cpu, idx, att, gnn, aux, r_out, r_e, r_aux, dtype=torch.float32):
-    """Run the oracle per channel; returns outputs and grads in the fused layout."""
+def oracle_layer_all(chs, x_cpu, idx, att, gnn, aux, r_out, r_e, r_aux, dtype=torch.float32, keep=None):
+    """Run the oracle per channel; returns outputs and grads in the fused layout.
+    keep: [E, C] dropout multipliers (the kernels' own mask, helpers.edge_keep) or None (no dropout).
+    r_e None: the loss has no edge_e term.  Output rows past r_out's (the halo sources of a rectangular
+    slice) are not destinations and are dropped."""
     p = {}
     for c, l in enumerate(chs):
         for name, prm in l.named_parameters():
             p["c%d.%s" % (c, name)] = prm.detach().cpu().clone().to(dtype).requires_grad_(True)
     x = x_cpu.clone().to(dtype).requires_grad_(True)
-    r_out, r_e, r_aux = r_out.to(dtype), r_e.to(dtype), [r.to(dtype) for r in r_aux]
+    r_out, r_aux = r_out.to(dtype), [r.to(dtype) for r in r_aux]
     outs, es, auxs = [], [], []
     for c in range(len(chs)):
-        o, e, au = od.disga_layer(p, "c%d." % c, x, idx, att, gnn, aux=aux)
+        o, e, au = od.disga_layer(p, "c%d." % c, x, idx, att, gnn, aux=aux,
+                                  keep=None if keep is None else keep[:, c:c + 1])
         outs.append(o)
         es.append(e)
         auxs.append(au)
-    out = torch.cat(outs, 1)
+    out = torch.cat(outs, 1)[:r_out.shape[0]]
     e = torch.cat(es, 1)
     au = [torch.cat([a_[k] for a_ in auxs], 1) for k in range(len(aux))]
-    loss = (out * r_out).sum() + (e * r_e).sum() + sum((a_ * r).sum() for a_, r in zip(au, r_aux))
+    loss = (out * r_out).sum() + sum((a_ * r).sum() for a_, r in zip(au, r_aux))
+    if r_e is not None:
+        loss = loss + (e * r_e.to(dtype)).sum()
     loss.backward()
     return out, e, au, x.grad, p
 
 
 CASES = [
-    # (n, m, C, D, F, max_chunk)
+    # (n, m, C, D, F, max_chunk[, kind])
     (300, 2500, 4, 64, 24, 16),     # VecT<2,16>, split rows
     (257, 1800, 8, 64, 100, 32),    # C=8 (config A shape), F=100
     (200, 1500, 2, 64, 16, 0),      # VecT<1,16>
@@ -244,38 +250,83 @@ CASES = [
     (260, 2200, 8, 64, 64, 16),     # F == D == 64: shared operand on the 128-bit layout (layer-2 shape), split rows
     (180, 1400, 4, 64, 64, 0),      # same, VecT<2,16>
     (150, 1000, 2, 64, 64, 8),      # same, VecT<1,16>
+    (200, 150, 4, 64, 16, 0, "sparse"),   # low degree; train mode at p = 0.9 drops every in-edge of some rows
+    (400, 3500, 8, 64, 20, 16, "slice"),  # middle destination range of a partition: rectangular, n_cols > n
 ]
+
+# (att, mode): train mode draws the dropout mask in the kernels (seed fixed below); "train-no-e" leaves
+# edge_e out of the loss, so the backward runs without a logit gradient (the benchmark's combination)
+ATT_MODES = [pytest.param(att, mode, id=str(att) if mode == "eval" else "%d-%s" % (att, mode))
+             for att, mode in [(1, "eval"), (1, "train"), (2, "eval"), (2, "train"), (3, "eval"), (3, "train"),
+                               (3, "train-no-e")]]
+SEED = 0xD1B54A32D192ED03     # both 32-bit halves of the seed enter the mask
+P_TRAIN = 0.3
+
+
+def slice_of(idx_np, n):
+    """Middle third of the destination rows of a square graph in a partition's local indexing
+    (own columns first, then halo), row-major sorted.  -> (indices, rows, columns)."""
+    from edgedisentangle_ssl_b200 import parallel as par
+    lo, hi = n // 3, 2 * n // 3
+    sel = (idx_np[0] >= lo) & (idx_np[0] < hi)
+    row_l, col_l, halo = par.compact_columns(lo, hi, idx_np[0][sel], idx_np[1][sel])
+    order = np.lexsort((col_l, row_l))
+    return np.stack([row_l[order], col_l[order]]), hi - lo, hi - lo + len(halo)
 
 
 @pytest.mark.parametrize("case", CASES)
-@pytest.mark.parametrize("att", [1, 2, 3])
+@pytest.mark.parametrize("att,mode", ATT_MODES)
 @pytest.mark.parametrize("gnn", ["AT", "GCN", "SAGE"])
-def test_fused_channels_vs_oracle(case, att, gnn):
-    n, m, C, D, Fin, max_chunk = case
+def test_fused_channels_vs_oracle(case, att, mode, gnn, monkeypatch):
+    from edgedisentangle_ssl_b200 import layers
+    from helpers import edge_keep
+    n, m, C, D, Fin, max_chunk = case[:6]
+    kind = case[6] if len(case) > 6 else None
+    train = mode != "eval"
+    p = (0.9 if kind == "sparse" else P_TRAIN) if train else 0.2
     torch.manual_seed(1000 + n + att)
     idx_np = hub_graph(n, m, seed=n)
+    n_cols = n
+    if kind == "slice":
+        idx_np, n, n_cols = slice_of(idx_np, n)
     idx = torch.from_numpy(idx_np)
     e_cnt = idx.shape[1]
-    chs = [edis.DisGALayer(Fin, D, dropout=0.2, alpha=0.1, att_type=att, gnn_type=gnn) for _ in range(C)]
-    x_cpu = torch.randn(n, Fin)
+    chs = [edis.DisGALayer(Fin, D, dropout=p, alpha=0.1, att_type=att, gnn_type=gnn) for _ in range(C)]
+    x_cpu = torch.randn(n_cols, Fin)
     rng = np.random.RandomState(7)
     aux = [torch.from_numpy(np.sort(rng.randint(0, n * n, 333))).long()]
     aux = [torch.stack([a_ // n, a_ % n]) for a_ in aux] + [torch.from_numpy(rng.randint(0, n, (2, 65))).long()]
     r_out, r_e = torch.randn(n, C * D), torch.randn(e_cnt, C)
     r_aux = [torch.randn(a_.shape[1], C) for a_ in aux]
-    o_ref, e_ref, au_ref, gx_ref, p_ref = oracle_layer_all(chs, x_cpu, idx, att, gnn, aux, r_out, r_e, r_aux)
-    _, _, _, gx_64, p_64 = oracle_layer_all(chs, x_cpu, idx, att, gnn, aux, r_out, r_e, r_aux, torch.float64)
+    if mode == "train-no-e":
+        r_e = None
+    keep = None
+    if train:
+        keep = edge_keep(SEED, e_cnt, C, p)
+        if kind == "sparse":
+            kept = np.zeros((n, C))
+            np.add.at(kept, idx_np[0], keep > 0)
+            assert (kept == 0).any(), "no (row, channel) pair with every in-edge dropped"
+        keep = torch.from_numpy(keep)
+    o_ref, e_ref, au_ref, gx_ref, p_ref = oracle_layer_all(chs, x_cpu, idx, att, gnn, aux, r_out, r_e, r_aux,
+                                                           keep=keep)
+    _, _, _, gx_64, p_64 = oracle_layer_all(chs, x_cpu, idx, att, gnn, aux, r_out, r_e, r_aux, torch.float64,
+                                            keep=keep)
 
+    monkeypatch.setattr(layers, "_next_seed", lambda: SEED)
     for l in chs:
-        l.to(DEV).eval()
-    graph = edis.Graph(n, idx_np[0], idx_np[1], device=DEV, max_chunk=max_chunk)
+        l.to(DEV).train(train)
+    graph = edis.Graph(n, idx_np[0], idx_np[1], device=DEV, max_chunk=max_chunk, n_cols=n_cols)
+    assert graph.info["was_sorted"]
     x = x_cpu.to(DEV).requires_grad_(True)
     out, e, au = run_channels(chs, x, graph, [a_.to(DEV) for a_ in aux])
     assert_close(out.cpu(), o_ref, RT, "out")
     assert_close(e.cpu(), e_ref, RT, "edge_e")
     for k in range(2):
         assert_close(au[k].cpu(), au_ref[k], RT, "aux%d" % k)
-    loss = (out * r_out.to(DEV)).sum() + (e * r_e.to(DEV)).sum() + sum((a_ * r.to(DEV)).sum() for a_, r in zip(au, r_aux))
+    loss = (out * r_out.to(DEV)).sum() + sum((a_ * r.to(DEV)).sum() for a_, r in zip(au, r_aux))
+    if r_e is not None:
+        loss = loss + (e * r_e.to(DEV)).sum()
     loss.backward()
     assert_close(x.grad.cpu(), gx_ref, grad_tol(gx_ref, gx_64), "gx")
     floor = group_floor([v.grad for v in p_ref.values() if v.grad is not None])
@@ -287,6 +338,35 @@ def test_fused_channels_vs_oracle(case, att, gnn):
                 assert prm.grad is None or float(prm.grad.abs().max()) == 0.0
             else:
                 assert_close(prm.grad.cpu(), ref, grad_tol(ref, p_64[key].grad), key, floor)
+
+
+@pytest.mark.parametrize("C", [2, 8, 16])
+@pytest.mark.parametrize("p", [0.1, 0.5, 0.9])
+@pytest.mark.parametrize("seed", [12345, SEED])
+def test_dropout_mask_matches_port(C, p, seed, monkeypatch):
+    """Every row has exactly one in-edge (CSR slot e = row e) and every V row is all-ones, so the
+    train-mode output is the mask itself: zero exactly where helpers.keep_scale drops, 1/(1-p) elsewhere.
+    C = 16 runs the LDG kernels with two channel groups; the agg plan runs the shared-operand kernels."""
+    from edgedisentangle_ssl_b200 import layers
+    from helpers import edge_keep
+    n, D, Fin = 4096, 64, 64
+    perm = np.random.RandomState(C).permutation(n)
+    graph = edis.Graph(n, np.arange(n), perm, device=DEV)
+    torch.manual_seed(C)
+    chs = [edis.DisGALayer(Fin, D, dropout=p, alpha=0.1, att_type=3, gnn_type="AT") for _ in range(C)]
+    for l in chs:
+        l.W_em.data.fill_(1.0 / Fin)
+        l.to(DEV).train()
+    monkeypatch.setattr(layers, "_next_seed", lambda: seed)
+    with torch.no_grad():
+        out, _, _ = run_channels(chs, torch.ones(n, Fin, device=DEV), graph)
+    out = out.reshape(n, C, D).cpu().numpy()
+    keep = edge_keep(seed, n, C, p)
+    assert np.array_equal(out == 0, np.broadcast_to((keep == 0)[:, :, None], out.shape))
+    kept = keep > 0
+    assert kept.any() and (~kept).any()
+    ref = np.broadcast_to(keep[:, :, None], out.shape)[kept]
+    assert np.abs(out[kept] - ref).max() <= 1e-6 * ref.max()
 
 
 def test_isolated_rows_and_empty_pairs():

@@ -285,3 +285,44 @@ def test_single_pass_softmax_backward_conditioning():
     one = max(rel_err(s32[k], g64[k], floor) for k in g64)
     print("fp32 vs float64, worst tensor: two-reduction form %.2e, single-pass form %.2e" % (two, one))
     assert two < 2e-5 and one < 1e-4
+
+
+# ------------------------------------------------------------------ the kernels' dropout mask, restated
+def test_dropout_mask_port_keep_rate_and_high_words():
+    """helpers.keep_scale (the numpy restatement the train-mode GPU tests build their oracle mask with):
+    keep rate 1 - p, multiplier float32 1 / (1 - p), and both 32-bit halves of the seed and of the
+    element index change the mask."""
+    from helpers import keep_scale
+    idx = np.arange(1 << 20, dtype=np.uint64)
+    seed = 0xD1B54A32D192ED03
+    for p in (0.1, 0.5, 0.9):
+        k = keep_scale(seed, idx, p)
+        assert k.dtype == np.float32
+        assert set(np.unique(k)) == {np.float32(0), np.float32(1) / (np.float32(1) - np.float32(p))}
+        assert abs((k > 0).mean() - (1 - p)) < 3e-3, p
+    base = keep_scale(seed, idx[:4096], 0.5) > 0
+    for other in (keep_scale(seed ^ (1 << 40), idx[:4096], 0.5), keep_scale(seed, idx[:4096] + np.uint64(1 << 33), 0.5),
+                  keep_scale(seed ^ 1, idx[:4096], 0.5)):
+        assert 0.4 < ((other > 0) != base).mean() < 0.6
+    assert np.array_equal(keep_scale(seed, idx[:4096], 0.5), keep_scale(seed, idx[:4096], 0.5))
+
+
+def test_oracle_keep_replaces_dropout():
+    """disga_layer(keep=...) multiplies alpha by the given mask: an all-kept mask of ones is the eval
+    result, and a mask that drops every in-edge of a row zeroes that row's AT output."""
+    torch.manual_seed(0)
+    n, fin, d = 30, 5, 4
+    idx = torch.from_numpy(og.build_adjacency(n, np.arange(n), (np.arange(n) + 1) % n)[0])
+    p = {"W": torch.randn(2 * fin, d), "a": torch.randn(d, 1), "W_em": torch.randn(fin, d)}
+    x = torch.randn(n, fin)
+    o0, e0 = od.disga_layer(p, "", x, idx, 3, "AT")
+    o1, e1 = od.disga_layer(p, "", x, idx, 3, "AT", keep=torch.ones(idx.shape[1], 1))
+    assert torch.equal(o0, o1) and torch.equal(e0, e1)
+    keep = torch.full((idx.shape[1], 1), 2.0)
+    keep[idx[0] == 3] = 0.0
+    o2, _ = od.disga_layer(p, "", x, idx, 3, "AT", keep=keep)
+    assert float(o2[3].abs().max()) == 0.0
+    rest = torch.arange(n) != 3
+    h0 = torch.where(o0 > 0, o0, torch.log1p(o0))     # inverse elu
+    h2 = torch.where(o2 > 0, o2, torch.log1p(o2))
+    assert torch.allclose(h2[rest], 2 * h0[rest], rtol=1e-5, atol=1e-6)
