@@ -1732,7 +1732,9 @@ extern "C" int edis_disga_sage_bwd(const edis_graph* g, const edis_layer_desc* d
                      (vec_ok(X, ldx) && vec_ok(neigh, 4) && vec_ok(g_neigh, 4) && vec_ok(gh, 4) && vec_ok(gX, 4)),
                  "edis_disga_sage_bwd: node tensors must be 16-byte aligned with ld %% 4 == 0");
   const int CD = d->C * d->D;
-  const int64_t pw = 2 * static_cast<int64_t>(CD) + 2 * d->C + d->Dv;
+  // rounded up to 4 floats: the 128-bit layouts store a split row's partials with float4 stores, so every
+  // slot must start 16-byte aligned (an odd F left odd slots misaligned)
+  const int64_t pw = (2 * static_cast<int64_t>(CD) + 2 * d->C + d->Dv + 3) / 4 * 4;
   if ((rc = check_ws(g, pw, workspace, workspace_bytes, "edis_disga_sage_bwd"))) return rc;
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   LayerArgs A = {};

@@ -212,8 +212,11 @@ __device__ __forceinline__ V ld_stream(const V* p) {
 // att-3 sign record: for each edge one bit per element of z = P_i + Q_j, bit set <=> z > 0.
 // The forward works on w = (-P_i) - Q_j = -z (negations are free operand modifiers) and pushes the
 // SIGN BIT of w into the record with one funnel shift per element, so element r of R ends up at bit
-// R-1-r.  (z == +0 from two +0 operands reads as positive; everything else, incl. exact cancellation
-// and -0, matches z > 0.  Such an edge carries no gradient to W in either case: x_i = x_j = 0.)
+// R-1-r.  (z == +0 from P_i = Q_j = +0 reads as positive (w = -0), where torch's leaky_relu takes the
+// 0.01 side; everything else, incl. an exact cancellation P_i = -Q_j != 0 (w = +0) and -0, matches
+// z > 0.  Both operands are +0 for all-zero rows x_i = x_j = 0, which carry no gradient to W, but also
+// when each dot product cancels exactly inside nonzero rows: there the element's gradient to W is taken
+// with slope 1 instead of 0.01.  Matching torch would cost an instruction per element.)
 __device__ __forceinline__ unsigned sign_push(unsigned mask, float w) {
   return __funnelshift_l(__float_as_uint(w), mask, 1);
 }

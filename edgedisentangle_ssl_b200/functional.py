@@ -292,7 +292,7 @@ def sage_backward_raw(graph, d, P, ldp, Q, ldq, X, a, agg, edge_e, stats, esign,
     gX = torch.empty(nc, Fin, dtype=torch.float32, device=dev) if need_gx else None
     edge_rec = _edge_rec(graph, d, dev)
     gh = torch.empty(n, C * Fin, dtype=torch.float32, device=dev)
-    ws, nbytes = _workspace(graph, 2 * CD + 2 * C + Fin, X)
+    ws, nbytes = _workspace(graph, (2 * CD + 2 * C + Fin + 3) // 4 * 4, X)   # 16-byte aligned partial rows
     base = d.flags
     plain = bool(base & _lib.FLAG_PLAIN_MEAN)
     fused_gx = bool(lib.edis_disga_sage_fused_gx(ctypes.byref(d)))

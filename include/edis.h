@@ -221,6 +221,8 @@ int edis_disga_sage_bwd(const edis_graph* g, const edis_layer_desc* d,
                         float* gP, int64_t ldgp, float* gQ, int64_t ldgq, float* ga, float* gX,
                         float* edge_rec, float* gh,
                         void* workspace, int64_t workspace_bytes, void* stream);
+/* edis_disga_sage_bwd: workspace >= edis_graph_workspace_bytes(g, W), W = 2*C*D + 2*C + F rounded up to a
+ * multiple of 4. */
 
 /* 1 if this shape runs on the 128-bit shared-operand path (F == D == 64, C in {2,4,8}), whose
  * source pass (EDIS_FLAG_PHASE_SRC) also produces gX: EDIS_FLAG_PHASE_GX is then a no-op. */
